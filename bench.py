@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- articles/sec of the DAE-with-triplet-loss training hot path (BASELINE.json metric).
 
-    python bench.py [--config C1|C2|C3|C4|C5] [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--config C1|C2|C3|C4|C5] [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one training step (corrupt -> encode -> decode -> loss -> triplet mining -> backward -> optimizer) on one batch of
 B = 800 articles.  Default workload = BASELINE.json configs[1] (C2): 100 000 synthetic articles per rank, 10 000-dim sparse TF-IDF
@@ -12,6 +12,10 @@ flat gradient per step).
 
 `--impl reference` times the reference algorithm restated on PyTorch-CPU (oracle/dae_oracle.py; TensorFlow 1.12 cannot be installed
 offline) on the host cores, same config.
+
+`--dump-outputs DIR` writes what the K-th step of the (first) timed window left to its caller -- the parameters enc_w, enc_b, dec_b
+and the step's scalars -- as DIR/<name>.npy.  Data, corruption and the epoch permutations are seeded, so the same arguments feed the
+same inputs and two runs agree to rounding (the kernels accumulate with float atomics).
 """
 import argparse
 import gc
@@ -56,7 +60,12 @@ def parse():
     ap.add_argument('--no-fit-api', action='store_true', help='skip the DenoisingAutoencoder.fit measurement')
     ap.add_argument('--no-graph', action='store_true', help='launch the step eagerly instead of replaying the captured CUDA graph')
     ap.add_argument('--cpu-steps', type=int, default=3)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the parameters and scalars of the last timed step as DIR/<name>.npy (same arguments, same inputs)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 def make_data(w, n_rows, seed):
@@ -252,6 +261,25 @@ def kernel_work(tag, w, s):
     return None, 0.0
 
 
+DUMP_W_BYTES = 60_000_000     # the encoder weights' share of the 64 MB that --dump-outputs may write
+
+
+def dump_outputs(dirname, F, H, theta, stats):
+    """What a caller of the training step holds after it: the updated parameters (float32) and the step's scalars (float64, the
+    slots of _cabi.STAT).  A weight matrix above DUMP_W_BYTES is written as a fixed, seeded sample of its rows (sorted)."""
+    os.makedirs(dirname, exist_ok=True)
+    theta = theta.cpu().numpy()
+    W = theta[:F * H].reshape(F, H)
+    out = {'enc_b': theta[F * H:F * H + H], 'dec_b': theta[F * H + H:], 'step_stats': stats.cpu().numpy()}
+    if W.nbytes <= DUMP_W_BYTES:
+        out['enc_w'] = W
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(F, DUMP_W_BYTES // W[0].nbytes, replace=False))
+        out['enc_w_row_sample'] = W[rows]
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+
 def batch_stats(w, x, labels, rng):
     """Per-batch figures of the algorithmic-work model, measured on one host-side sample batch."""
     B = w['B']
@@ -306,10 +334,12 @@ def main():
     steps_per_epoch = n_rows // B
     perm_buf = torch.zeros(n_rows, dtype=torch.int32, device=dev)
     use_graph = not args.no_graph
+    perm_gen = torch.Generator(device=dev)
+    perm_gen.manual_seed(4321 + rank)        # the default CUDA generator is seeded differently in every process
 
     def epoch_start(epoch):
         eng.corrupt_masking(w['corr_frac'], seed=1234 + rank, epoch=epoch)           # utils.masking_noise, on device
-        perm_buf.copy_(torch.randperm(n_rows, device=dev, dtype=torch.int32))         # utils.gen_batches shuffle
+        perm_buf.copy_(torch.randperm(n_rows, device=dev, dtype=torch.int32, generator=perm_gen))   # utils.gen_batches shuffle
 
     def eager_step(offset, log_row):
         if explicit:
@@ -401,6 +431,8 @@ def main():
 
     ms, gpu_launches, clk = timed_window(first)
     losses = log.cpu().numpy()
+    # the first window's K-th step: its inputs do not depend on whether a host-stalled window is re-measured below
+    last_step = (eng.theta.clone(), log[K - 1].clone()) if args.dump_outputs else None
     prof = profile(first + K)
     # validity guard: the overlapped step cannot take longer than its kernels run one after another on ONE stream (`prof`, device time)
     # plus the gradient exchange.  A window above 1.25x that bound had the GPU idle waiting for the host (a stalled launch call: seen
@@ -536,6 +568,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, F, H, *last_step)
 
     cpu_baseline = None
     if not args.no_cpu_baseline:

@@ -122,13 +122,36 @@ def test_data_dir_cache_round_trip(tmp_path):
     assert list(lab.columns) == ['label_story', 'label_category_publish_name', 'title', 'story', 'category_publish_name'] and len(lab) == 40
 
 
-@pytest.mark.skipif(not os.path.isfile('/root/reference/datasets/uci_news.snappy.parquet'), reason='UCI corpus only in the builder container')
 def test_uci_preparation_matches_the_reference_configuration(tmp_path):
-    """C1 of BASELINE.json: 8000 x 10000 binary CSR from the UCI corpus (SURVEY 8d quotes nnz 1 241 293)."""
+    """C1 of BASELINE.json: 8000 x 10000 binary CSR from the UCI corpus (SURVEY 8d quotes nnz 1 241 293).  The preparation runs on
+    the newest 300 articles of the corpus (tests/golden/uci_news_sample.parquet) and must give exactly what the reference's own
+    vectoriser gives (tests/golden/uci_prep_sample.npz, oracle/gen_golden_uci_sample.py); the full-size matrices are the
+    committed fixture tests/golden/uci_c1.npz, which the same preparation wrote from the whole corpus with the default flags."""
     import main_autoencoder as cli
-    F = cli.check_flags(cli.build_parser().parse_args(['--model_name', 'uci', '--data_path', '/root/reference/datasets/uci_news.snappy.parquet']))
+    from helpers import load_uci_c1
+    gold = np.load(os.path.join(ROOT, 'tests', 'golden', 'uci_prep_sample.npz'))
+    F = cli.check_flags(cli.build_parser().parse_args([
+        '--model_name', 'uci', '--data_path', os.path.join(ROOT, 'tests', 'golden', 'uci_news_sample.parquet'),
+        '--train_row', str(int(gold['train_row'])), '--validate_row', str(int(gold['validate_row'])),
+        '--max_features', str(int(gold['max_features']))]))
     d = cli.prepare_uci(F, None)
-    X, Xv = d['binary']
+    assert list(d['count_vectorizer'].get_feature_names_out()) == list(gold['vocabulary'])
+    for k, split in enumerate(('train', 'validate')):
+        X, Xt = d['binary'][k].tocsr(), d['tfidf'][k].tocsr()
+        X.sort_indices()
+        Xt.sort_indices()
+        assert X.shape == tuple(gold[split + '_shape'])
+        assert (X.indptr == gold[split + '_indptr']).all() and (X.indices == gold[split + '_indices']).all()
+        assert (X.data == 1).all() and (Xt.indptr == X.indptr).all() and (Xt.indices == X.indices).all()
+        assert np.allclose(Xt.data, gold[split + '_tfidf'], rtol=1e-12, atol=0)
+        assert (d['articles' if k == 0 else 'articles_validate'].article_id.values == gold[split + '_article_id']).all()
+        for lab in ('category_publish_name', 'story'):
+            assert (np.asarray(d['label_' + lab][k]) == gold['%s_label_%s' % (split, lab)]).all(), (split, lab)
+
+    defaults = cli.check_flags(cli.build_parser().parse_args(['--model_name', 'uci']))
+    assert (defaults.train_row, defaults.validate_row, defaults.max_features) == (8000, 2000, 10000)
+    full = load_uci_c1()
+    X, Xv = full['train'], full['validate']
     assert X.shape == (8000, 10000) and Xv.shape == (2000, 10000)
     assert abs(X.nnz - 1241293) <= 0.01 * 1241293
-    assert len(np.unique(d['label_category_publish_name'][0])) == 4
+    assert len(np.unique(full['train_label_category_publish_name'])) == 4
